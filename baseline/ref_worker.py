@@ -3,7 +3,7 @@
 dumped as .npy files -- the same arrays the GPU arm multiplies.
 
     python baseline/ref_worker.py numba <dir> <steps> <warmup>
-        The UNMODIFIED reference (baseline/_ref, installed by tools/make_ref.sh): runs with PYTHONPATH=baseline/_ref so
+        The UNMODIFIED reference (oracle/_ref, installed by oracle/make_ref.sh): runs with PYTHONPATH=oracle/_ref so
         that `import sparse` is pydata/sparse's numba backend, in a process of its own (the product package never shares
         an interpreter with the reference).  The timed call is the reference's public API for the path,
         `sparse.tensordot(GCXS, ndarray, axes=1)` (numba_backend/_common.py:95 -> _dot :339 -> _dot_csr_ndarray
@@ -35,7 +35,7 @@ def main():
     info = {}
     if impl == "numba":
         import numba
-        import sparse  # the reference (PYTHONPATH=baseline/_ref)
+        import sparse  # the reference (PYTHONPATH=oracle/_ref)
 
         A = sparse.GCXS((data, indices, indptr), shape=shape, compressed_axes=(0,))
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the hot path (BASELINE.json: configs[1] = C2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--gather ce|nccl]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--gather ce|nccl] [--dump-outputs DIR]
 
 Workload C2: GCXS/CSR A (1e6 x 1e6, nnz 1e8, fp32, uniform-random positions) times dense
 B (1e6 x 128 fp32) -> dense C, i.e. ``sparse.tensordot(A, B, axes=1)`` -> _dot_csr_ndarray
@@ -12,7 +12,7 @@ B (1e6 x 128 fp32) -> dense C, i.e. ``sparse.tensordot(A, B, axes=1)`` -> _dot_c
                pinned host arrays in, host array out, H2D/D2H inside the timed region.
 * ``roofline`` algorithmic bytes (gather model, SURVEY.md s8(d): 525 B/nnz with int32 indices)
                / measured kernel time, against MEASURED_PEAKS.json's HBM copy bandwidth.
-* ``cpu_baseline``  the REFERENCE ITSELF -- pydata/sparse's numba path (baseline/_ref, tools/make_ref.sh), called as
+* ``cpu_baseline``  the REFERENCE ITSELF -- pydata/sparse's numba path (oracle/_ref, oracle/make_ref.sh), called as
                sparse.tensordot(GCXS, ndarray, axes=1) in a worker process (baseline/ref_worker.py), 1 core (the
                kernel is single-threaded by construction) -- on the first 1e5 rows of the very arrays the GPU
                multiplies, its output bit-compared with the GPU's rows; plus a labelled all-cores figure from the
@@ -26,6 +26,13 @@ B (1e6 x 128 fp32) -> dense C, i.e. ``sparse.tensordot(A, B, axes=1)`` -> _dot_c
 
 Inputs are synthetic (seeded torch generators on the device); 2.2 GB of operands per rank is far
 larger than the 126 MB L2, so no explicit L2 flush is needed between steps ("l2": "inputs>L2").
+
+``--dump-outputs DIR`` writes what the timed path returned in its last step: ``C.npy`` (float32) holds rows of C and
+``C_rows.npy`` (float64) their row indices -- all rows when C fits in 64 MB, else a fixed seeded sample of rows.  With
+the same arguments the inputs are the same on every run, so two builds can be compared output for output.  With N > 1
+(weak scaling: every rank multiplies its OWN M-row matrix A, seeded A_SEED + rank) every rank writes ``C_rank<r>.npy``
+/ ``C_rows_rank<r>.npy`` for its own product, within 64 MB / N; the row indices are local to that product, so the files
+are N separate results, not blocks of one C.
 """
 from __future__ import annotations
 
@@ -61,7 +68,12 @@ def parse():
     p.add_argument("--no-strong", action="store_true", help="N>1: skip the strong-scaling block")
     p.add_argument("--no-configs", action="store_true", help="N=1: skip the per-config block (C1, C3, C4, C5, ...)")
     p.add_argument("--no-numa", action="store_true", help="do not pin the process to the GPU's NUMA node")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write C of the last timed step (or a seeded row sample of it, 64 MB at most) as .npy files")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------
@@ -204,8 +216,27 @@ def algorithmic_bytes(nnz, M, ncols, vb=4, ib=4):
     return nnz * (vb + ib) + (M + 1) * ib + nnz * ncols * vb + M * ncols * vb
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs: payload of all files together (the .npy headers fit in the slack)
+DUMP_SEED = 2024
+
+
+def dump_rows(M, ncols, share=1):
+    """Rows of an M x ncols fp32 C that --dump-outputs writes: all of them when they fit in DUMP_BYTES / share, else a
+    fixed seeded sample (sorted), the same on every run.  Each row costs ncols * 4 bytes of C + 8 for its index."""
+    n = DUMP_BYTES // share // (ncols * 4 + 8)
+    if M <= n:
+        return np.arange(M)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(M, size=n, replace=False))
+
+
+def write_outputs(d, c_rows, rows, suffix=""):
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, f"C{suffix}.npy"), np.ascontiguousarray(c_rows, dtype=np.float32))
+    np.save(os.path.join(d, f"C_rows{suffix}.npy"), rows.astype(np.float64))
+
+
 # ---- CPU legs: the reference (numba) and the OpenMP port, each in a worker process, on dumped arrays -------------------
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 WORKER = os.path.join(ROOT, "baseline", "ref_worker.py")
 CPU_ROWS = 100_000      # rows of A in the CPU sample (x full B): ~1e7 nnz, ~0.5 s per numba call
 PORT_THREADS = 32       # fixed; does not follow OMP_NUM_THREADS (torchrun exports 1)
@@ -256,10 +287,11 @@ def run_worker(impl, d, steps, warmup, threads=None, timeout=900):
         return json.load(f)
 
 
-def cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps, warmup, gpu_rows=None):
+def cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps, warmup, gpu_rows=None, dump_dir=None):
     """Time the reference (numba, 1 core) and the port (fixed threads) on the same dumped sample.  Returns the
     `cpu_baseline` object; when `gpu_rows` (the GPU's C[:rows_sample] as a host array) is given, both outputs are
-    bit-compared with it."""
+    bit-compared with it.  `dump_dir`: write the last result of the reference (of the port when the reference is not
+    installed) there, as --dump-outputs does."""
     import shutil
 
     d, n = dump_sample(vals, cols, indptr, B, rows_sample, K)
@@ -279,7 +311,7 @@ def cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps, warmup, gpu_ro
                 out["parity_bit_exact_vs_gpu"] = bool(c.shape == gpu_rows.shape and np.array_equal(
                     c.view(np.uint32), gpu_rows.view(np.uint32)))
         threads = min(PORT_THREADS, os.cpu_count() or 1)
-        r = run_worker("port", d, max(steps, 3), max(warmup, 1), threads=threads)
+        r = run_worker("port", d, steps, max(warmup, 1), threads=threads)
         med = float(np.median(r["seconds"]))
         port = {"value": round(n / med / 1e9, 5), "unit": "GNNZ/s", "cores": r["threads"], "kind": "port",
                 "best": round(n / min(r["seconds"]) / 1e9, 5),
@@ -289,8 +321,12 @@ def cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps, warmup, gpu_ro
             port["parity_bit_exact_vs_gpu"] = bool(np.array_equal(c.view(np.uint32), gpu_rows.view(np.uint32)))
         if out:
             out["all_cores_port"] = port
-        else:  # baseline/_ref was not shipped: the port is all there is (and says so)
-            out = dict(port, sample=sample + "; baseline/_ref missing (run tools/make_ref.sh), so this is the C port")
+        else:  # oracle/_ref is not installed: the port is all there is (and says so)
+            out = dict(port, sample=sample + "; oracle/_ref missing (see oracle/make_ref.sh), so this is the C port")
+        if dump_dir is not None:
+            c = np.load(os.path.join(d, "C_numba.npy" if out["kind"] == "reference" else "C_port.npy"))
+            rows = dump_rows(c.shape[0], c.shape[1])
+            write_outputs(dump_dir, c[rows], rows)
         return out
     finally:
         shutil.rmtree(d, ignore_errors=True)
@@ -482,6 +518,10 @@ def main():
     launches0 = _lib.launch_count()
     ms_per_step, kern_ms, clk = timed(run_steps, args.steps, clock_index=sampler)
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs is not None:  # C still holds the last timed step; the blocks below reuse it
+        rows = dump_rows(M, ncols, share=world)
+        write_outputs(args.dump_outputs, C[torch.from_numpy(rows).to(dev)].cpu().numpy(), rows,
+                      suffix=f"_rank{rank}" if world > 1 else "")
     nnz_all = allsum(nnz)
     value = nnz_all / (ms_per_step * 1e-3) / 1e9
 
@@ -547,7 +587,7 @@ def main():
         import sparse_b200 as sp
 
         npv = (h_vals.numpy(), h_cols.numpy(), h_ptr.numpy(), h_B.numpy())
-        esteps = max(3, min(args.steps, 10))
+        esteps = args.steps
 
         def e2e_step():
             # the call a user of the reference makes: host arrays in, np.ndarray out (H2D + K1 + D2H inside)
@@ -652,7 +692,7 @@ def workload_config(M, K, nnz, ncols, world, gather_kind=None):
 def reference_arm(args, rank, local_rank, world):
     """--impl reference: the reference's OWN implementation of the path on the host cores.
 
-    baseline/_ref holds the unmodified pydata/sparse (tools/make_ref.sh); a worker process imports it and times
+    oracle/_ref holds the unmodified pydata/sparse (oracle/make_ref.sh); a worker process imports it and times
     `sparse.tensordot(GCXS, ndarray, axes=1)` -> _dot_csr_ndarray (_common.py:95, 720-755), a single-threaded numba
     kernel (cores = 1 by construction), on a bounded sample of the GPU arm's own arrays: the first CPU_ROWS rows of
     rank 0's A (same seeded generator, run on cuda:0 when the box has one -- input generation only) times the full B.
@@ -671,7 +711,8 @@ def reference_arm(args, rank, local_rank, world):
     else:  # authoring container: same distribution, host generator, only the sampled rows
         vals, cols, indptr, _ = gen_A(torch, rows_sample, K, args.nnz // max(1, M // rows_sample), A_SEED, dev)
     B = gen_B(torch, K, ncols, B_SEED, dev)
-    cpu = cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps=args.steps, warmup=max(args.warmup, 1))
+    cpu = cpu_legs(vals, cols, indptr, B, K, ncols, rows_sample, steps=args.steps, warmup=max(args.warmup, 1),
+                   dump_dir=args.dump_outputs)
     val = cpu["value"]
     n = int(indptr[rows_sample].item())
     line = {

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Differential fuzzing of the ORACLE (oracle/dot_oracle.c, the CPU restatement the GPU parity tests compare with)
-against the reference's own numba kernels -- authoring container only (needs baseline/_ref, tools/make_ref.sh).
+against the reference's own numba kernels; needs the reference installed in oracle/_ref (oracle/make_ref.sh).
 
     python tools/fuzz_oracle_vs_reference.py [--cases 400] [--seed 0]
 
@@ -22,7 +22,7 @@ import warnings
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
+sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))
 sys.path.insert(0, ROOT)
 
 import sparse as R  # noqa: E402
