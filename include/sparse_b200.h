@@ -287,6 +287,17 @@ int b2s_mttkrp(int dtype, int idx_bytes, int64_t I_, int64_t J, const void *indp
                const void *l_dev, const void *vals_dev, const void *d_dev, int64_t ldd, const void *c_dev, int64_t ldc,
                void *out_dev, int64_t ldo, void *stream);
 
+/* ---- masked sparse product (K10, masked_spgemm.cu) ----------------------------------------- */
+/* examples/triangles_example.py `a @ a * a`, i.e. s * (a @ b) with sparse a and b, without forming a @ b:
+ * out_vals[p] = s_vals[p] * sum_k A[i_p,k] * Bt[j_p,k] over the k stored in both rows, summed in ascending k.  S, A and
+ * Bt (b compressed by column) are CSR with sorted rows; s_vals / out_vals are dtype_out, a_data / bt_data dtype_ab.
+ * Pairs (dtype_ab, dtype_out): (F32,F32) (F32,F64) (F64,F64) (I64,I64) (I64,F64) (BOOL, BOOL|I64|F32|F64). */
+int b2s_masked_spgemm(int dtype_ab, int dtype_out, int idx_bytes, int64_t M, int64_t N, int64_t K,
+                      const void *s_indptr_dev, const void *s_cols_dev, const void *s_vals_dev,
+                      const void *a_indptr_dev, const void *a_indices_dev, const void *a_data_dev,
+                      const void *bt_indptr_dev, const void *bt_indices_dev, const void *bt_data_dev,
+                      void *out_vals_dev, void *stream);
+
 /* ---- copy-engine exchange of a row-sharded dense operand (peer.cu; SURVEY.md s8(e), no reference counterpart: the
  * reference is single-process) ------------------------------------------------------------------------------------
  * b2s_peer_alloc: cudaMalloc'ed (IPC-exportable) device buffer; b2s_peer_export writes its 64-byte CUDA IPC handle;

@@ -2,7 +2,8 @@
 
 Drop-in names for that path: ``COO``, ``GCXS`` (``CSR``/``CSC``), ``tensordot``, ``matmul``, ``dot``,
 ``elemwise``, reductions (``sum``/``max``/``min``/``prod``/``mean``/``any``/``all`` and the ``nan*`` forms) and the NumPy protocols
-(``__array_ufunc__``, ``__array_function__``, ``@``), plus the fused ``sddmm`` and ``mttkrp`` example paths.
+(``__array_ufunc__``, ``__array_function__``, ``@``), plus the fused ``sddmm`` and ``mttkrp`` example paths and the masked sparse product
+``masked_matmul(s, a, b)`` = ``s * (a @ b)`` for sparse ``a``, ``b``.
 Host code is Python; every data-path step is a hand-written CUDA kernel in ``libsparse_b200.so`` reached through a
 thin C ABI (``include/sparse_b200.h``) via ctypes.  There is no CPU fallback: without the library or a CUDA device
 operations raise.
@@ -39,7 +40,7 @@ from ._dok import DOK
 from ._dot import dot, matmul, tensordot
 from ._einsum import einsum
 from ._elemwise import broadcast_to, elemwise, where
-from ._fused import mttkrp, sddmm
+from ._fused import masked_matmul, mttkrp, sddmm
 from ._gcxs import CSC, CSR, GCXS
 from ._io import load_npz, save_npz
 from ._manip import (concatenate, diagonal, diagonalize, expand_dims, flip, kron, matrix_transpose, moveaxis, outer,
@@ -50,8 +51,8 @@ from ._sorting import sort, unique_counts, unique_values
 from ._sparse_array import SparseArray
 
 __version__ = "0.1.0"
-# `__all__` below is exactly upstream's namespace (tests/test_namespace.py there); the fused example kernels `sddmm` and
-# `mttkrp`, the 2-D classes `CSR` / `CSC` and a few helpers are importable attributes outside of it.
+# `__all__` below is exactly upstream's namespace (tests/test_namespace.py there); the fused example kernels `sddmm`,
+# `mttkrp` and `masked_matmul`, the 2-D classes `CSR` / `CSC` and a few helpers are importable attributes outside of it.
 
 
 def clip(a, min=None, max=None, out=None):

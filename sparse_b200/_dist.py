@@ -7,6 +7,7 @@ only exchange is making the right operand visible to every rank (SURVEY.md s8(e)
   all-gathered over NCCL/NVLink (``dist.all_gather_into_tensor``) before the local K1 kernel.
 * ``spgemm_rowblock``      C_r = A_r @ B for sparse B: B's CSR arrays are all-gathered (variable sizes, padded).
 * ``sddmm_rowblock``       mask row block x local rows of `a`; `b` (K x N) arrives column-sharded and is gathered.
+* ``masked_matmul_rowblock`` sparse mask row block x local rows of sparse `a`; `b`'s row blocks (CSR) are gathered.
 
 No reduction collective is needed for row blocking (a reduce-scatter would only appear if the CONTRACTION axis
 were split, which doubles the dense traffic; see DESIGN.md).  Host logic is backend-agnostic: the `gloo` tests
@@ -428,6 +429,15 @@ def sddmm_rowblock(s_local, a_local, b_cols_shard, group=None):
     bt_shard = Kn.transpose_dense(b_cols_shard)  # (N/world, K)
     Bt = all_gather_rows(bt_shard, group)        # (N, K)
     return sddmm(s_local, a_local, Bt, b_transposed=True)
+
+
+def masked_matmul_rowblock(s_local, a_local, b_local, group=None):
+    """Local row block of ``s * (a @ b)`` for sparse operands: `s` and `a` hold the same block of rows, `b` is
+    row-sharded as CSR blocks that are all-gathered, then K10 runs locally."""
+    from ._fused import masked_matmul
+
+    B = gather_csr_rows(b_local, group)
+    return masked_matmul(s_local, a_local, B)
 
 
 # ---- element-wise operations and reductions: range partition on the leading coordinate (SURVEY.md s8(e)) -------------

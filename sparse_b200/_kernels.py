@@ -641,3 +641,23 @@ def mttkrp(indptr, kk, ll, vals, Dm, Cm, I_, J):
                                i64(J), vp(D.ptr(out)), i64(J), _sp())
     _lib.check(rc, "b2s_mttkrp")
     return out
+
+
+# ------------------------------------------------------------------------------------------------
+# K10 masked sparse product
+# ------------------------------------------------------------------------------------------------
+def masked_spgemm(s_indptr, s_cols, s_vals, a_indptr, a_indices, a_data, bt_indptr, bt_indices, bt_data, M, N, K):
+    """out_vals[p] = s_vals[p] * sum_k a[i_p, k] * bt[j_p, k], ascending k  (`s * (a @ b)` of
+    examples/triangles_example.py without the product).  All index arrays share one dtype."""
+    t = _t()
+    dt_ab = D.np_dtype(a_data)
+    assert bt_data.dtype == a_data.dtype
+    assert all(x.dtype == s_indptr.dtype for x in (s_cols, a_indptr, a_indices, bt_indptr, bt_indices))
+    out = t.empty_like(s_vals)
+    rc = _lib.load().b2s_masked_spgemm(i32(D.dtype_code(dt_ab)), i32(D.dtype_code(D.np_dtype(s_vals))),
+                                      i32(_idx_bytes(s_indptr)), i64(M), i64(N), i64(K), vp(D.ptr(s_indptr)),
+                                      vp(D.ptr(s_cols)), vp(D.ptr(s_vals)), vp(D.ptr(a_indptr)), vp(D.ptr(a_indices)),
+                                      vp(D.ptr(a_data)), vp(D.ptr(bt_indptr)), vp(D.ptr(bt_indices)),
+                                      vp(D.ptr(bt_data)), vp(D.ptr(out)), _sp())
+    _lib.check(rc, "b2s_masked_spgemm")
+    return out
